@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """bench.py — block-sparse attention at HunyuanVideo 720p (BASELINE.json metric / configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes the output of the last timed step, sampled at fixed token rows, to DIR/out.npy
+(see dump_outputs), so that two builds run with the same arguments can be compared output for output.
 
 One step = one pass of the SVG1 sparse attention core over synthetic Q/K/V of the HunyuanVideo 720p
 shape (B=1, H=24, S=119056 = 33 frames x 3600 tokens + 256 text, D=128, bf16) under the executed SVG1
@@ -36,6 +39,7 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 sys.path.insert(0, str(ROOT / "sparse-videogen_b200"))
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ for the modules imported from it
 
 import torch  # noqa: E402
 
@@ -44,6 +48,19 @@ H_TOTAL, D, CTX, F, P, PROMPT_LEN = 24, 128, 256, 33, 3600, 60
 S = CTX + F * P
 SPARSITY = 0.30
 N_SAMPLED_ROWS, SAMPLE_MAX_ROW = 64, 10000
+DUMP_ROWS = 2048  # token rows kept by --dump-outputs: 24 heads x 2048 x 128 fp32 = 25 MB instead of 1.5 GB
+
+
+def dump_outputs(out_dir, o):
+    """Write the attention output o [1, H, S, D] at DUMP_ROWS token rows drawn once from a fixed seed (sorted) as
+    <out_dir>/out.npy, float32 [H, DUMP_ROWS, D]."""
+    import numpy as np
+
+    rows = torch.randperm(S, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    sample = o[0].index_select(1, rows.to(o.device)).float().cpu().numpy()
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "out.npy", sample)
 
 
 def band_width(sparsity=SPARSITY):
@@ -405,7 +422,8 @@ def run_ours(args):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step(timed=True)
+        out = None  # release the previous step's output before this step allocates, as in the warmup steps
+        out = step(timed=True)
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
@@ -422,6 +440,9 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_step = t[0].item() / args.steps
     attn_ms = t[1].item()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
+    del out
 
     # ---- output checksum on FIXED sampled rows: must be identical for every N (heads are generated per global id,
     # per-head computation does not depend on the sharding) -> compare across the lines of a scaling run
@@ -566,7 +587,8 @@ def run_ours(args):
     if world == 1 and not args.no_ref_gpu and not args.no_extras:
         try:
             r = subprocess.run([sys.executable, str(ROOT / "tools" / "ref_gpu_paths.py"), "--heads", str(H_TOTAL)],
-                               capture_output=True, text=True, timeout=args.ref_gpu_timeout)
+                               capture_output=True, text=True, timeout=args.ref_gpu_timeout,
+                               env=dict(os.environ, PYTHONDONTWRITEBYTECODE="1"))
             for ln in r.stdout.splitlines():
                 if ln.startswith("REF_GPU_JSON "):
                     ref_gpu = json.loads(ln[len("REF_GPU_JSON "):])
@@ -634,7 +656,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="headline + roofline + e2e only (skip SVG2 pipeline, FP8 sweep, ref_gpu)")
     ap.add_argument("--no-ref-gpu", action="store_true", help="skip timing the reference's own GPU paths")
     ap.add_argument("--ref-gpu-timeout", type=float, default=420.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's output, sampled at fixed token rows, to DIR/out.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,6 +1,7 @@
 """Seeded input generators shared by the golden-vector scripts and the tests that consume the vectors, so that large
 random inputs are stored as (seed, checksum) instead of raw tensors.  torch's CPU generator is bit-reproducible for a
 given torch build (the GPU box runs the same image); every consumer checks the stored checksum first."""
+import numpy as np
 import torch
 
 
@@ -57,6 +58,28 @@ def structured_qkv(seed, H, F, P, ctx, D, text_first=False, scale=1.5):
         q[0, h, lo:lo + V] += emb[idx]
         k[0, h, lo:lo + V] += emb[idx]
     return q.bfloat16(), k.bfloat16(), v.bfloat16()
+
+
+KM_FULLSIZE = ("hyq", "hyk", "wank")  # k-means cases at the HunyuanVideo / Wan token counts
+KM_GOLDEN = ("kmeans_golden.npz", "kmeans_golden_fullsize.npz")  # two files so that neither exceeds 1 MB
+
+
+def split_kmeans_golden(out):
+    """{name: array} -> the two dicts stored as KM_GOLDEN: the full-size cases go to the second file."""
+    full = {k: v for k, v in out.items() if k.startswith("km_") and k.split("_")[1] in KM_FULLSIZE}
+    return {k: v for k, v in out.items() if k not in full}, full
+
+
+def load_kmeans_golden(golden_dir):
+    """Both KM_GOLDEN files merged into one {name: array} dict, or None when they have not been generated."""
+    paths = [golden_dir / n for n in KM_GOLDEN]
+    if not all(p.exists() for p in paths):
+        return None
+    out = {}
+    for p in paths:
+        with np.load(p) as z:
+            out.update({k: z[k] for k in z.files})
+    return out
 
 
 DM_CASES = {"hy": (2, 400, 1000, 128), "small": (3, 12, 40, 64)}

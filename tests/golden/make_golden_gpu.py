@@ -25,7 +25,7 @@ HERE = Path(__file__).resolve().parent
 ROOT = HERE.parents[1]
 sys.path.insert(0, str(HERE))
 import ref_import as R  # noqa: E402
-from gen_inputs import DM_CASES, checksum, dm_inputs, kmeans_inputs  # noqa: E402
+from gen_inputs import DM_CASES, KM_GOLDEN, checksum, dm_inputs, kmeans_inputs, split_kmeans_golden  # noqa: E402
 
 BIG = ("hyq", "hyk", "wank")  # full-size cases: big arrays are stored subsampled (every 4th token / centroid)
 
@@ -130,8 +130,9 @@ def main():
 
     dst = ROOT / "gpurun_out"
     dst.mkdir(exist_ok=True)
-    np.savez_compressed(dst / "kmeans_golden.npz", **out)
-    print("wrote", dst / "kmeans_golden.npz")
+    for name, part in zip(KM_GOLDEN, split_kmeans_golden(out)):
+        np.savez_compressed(dst / name, **part)
+        print("wrote", dst / name)
 
 
 if __name__ == "__main__":

@@ -1,9 +1,10 @@
 """Import helpers for the UNMODIFIED reference.
 
-Two places can hold it: the read-only checkout `/root/reference` (build container only) and the git-ignored
-install `baseline/_ref` (written by tools/install_reference.py; it travels to the GPU box with the snapshot,
-which is how the reference's Triton / FlashInfer code is executed on a B200 for golden vectors and for
-bench.py's `ref_gpu` section).  Nothing in the product package imports this module.
+The reference is not part of this repository.  Two places can hold it: a Sparse-VideoGen checkout named by the
+environment variable SVGB200_REFERENCE and the git-ignored install `baseline/_ref` (written by
+tools/install_reference.py), which is how the reference's Triton / FlashInfer code is executed on a B200 for
+golden vectors and for bench.py's `ref_gpu` section.  Without either, the tests that import it skip.  Nothing in
+the product package imports this module.
 
 Packages the reference imports at module scope but that this image lacks are replaced by inert stubs — none of
 them is touched by the functions we execute:
@@ -17,7 +18,7 @@ import types
 from pathlib import Path
 
 ROOT = Path(__file__).resolve().parents[2]
-CANDIDATES = ["/root/reference", str(ROOT / "baseline" / "_ref")]
+CANDIDATES = [p for p in (os.environ.get("SVGB200_REFERENCE"), str(ROOT / "baseline" / "_ref")) if p]
 
 
 def reference_root():
@@ -84,7 +85,7 @@ def install_stubs():
 def _path():
     root = reference_root()
     if root is None:
-        raise ImportError("the reference is neither mounted at /root/reference nor installed in baseline/_ref "
+        raise ImportError("the reference is neither named by SVGB200_REFERENCE nor installed in baseline/_ref "
                           "(python tools/install_reference.py)")
     if root not in sys.path:
         sys.path.insert(0, root)

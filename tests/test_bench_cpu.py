@@ -28,6 +28,27 @@ def test_cpu_sample_is_time_boxed():
     assert "256 query rows" in sample
 
 
+def test_dump_outputs_writes_a_fixed_float32_row_sample(tmp_path):
+    sys.path.insert(0, str(ROOT))
+    import bench
+    import numpy as np
+    import torch
+
+    o = torch.randn(1, 2, bench.S, 4, generator=torch.Generator().manual_seed(3)).bfloat16()
+    bench.dump_outputs(tmp_path / "a", o)
+    bench.dump_outputs(tmp_path / "b", o)
+    a, b = np.load(tmp_path / "a" / "out.npy"), np.load(tmp_path / "b" / "out.npy")
+    assert a.dtype == np.float32 and a.shape == (2, bench.DUMP_ROWS, 4) and np.array_equal(a, b)
+    rows = [int(np.flatnonzero((o[0, 0].float().numpy() == a[0, i]).all(-1))[0]) for i in (0, -1)]
+    assert rows[0] < rows[1] and np.array_equal(a[:, -1], o[0, :, rows[1]].float().numpy())
+
+
+def test_steps_must_be_positive():
+    out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=120, cwd=ROOT)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
 def test_reference_arm_prints_the_contract_line():
     env = dict(os.environ, RANK="0")
     out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],

@@ -1,7 +1,7 @@
 """The drop-in, proven against the REAL reference processors.
 
-The unmodified reference is imported (tests/golden/ref_import.py: /root/reference in the build container, the
-git-ignored install baseline/_ref on the GPU box; `diffusers` / `cuvs` replaced by inert stubs),
+The unmodified reference is imported (tests/golden/ref_import.py: a checkout named by SVGB200_REFERENCE or the
+git-ignored install baseline/_ref; `diffusers` / `cuvs` replaced by inert stubs),
 `svgb200.patch.install(module)` swaps the operator names the reference resolves as module globals, and the
 reference's OWN `attention_core_logic` runs on the GPU:
 
@@ -24,7 +24,7 @@ sys.path.insert(0, str(HERE / "golden"))
 import ref_import as R  # noqa: E402
 from gen_inputs import structured_qkv  # noqa: E402
 
-needs_ref = pytest.mark.skipif(not R.reference_available(), reason="reference not importable (no /root/reference, no baseline/_ref)")
+needs_ref = pytest.mark.skipif(not R.reference_available(), reason="reference not importable (no SVGB200_REFERENCE, no baseline/_ref)")
 
 
 def _positional(fn):

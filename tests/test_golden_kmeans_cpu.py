@@ -10,13 +10,12 @@ import torch
 
 HERE = Path(__file__).resolve().parent
 sys.path.insert(0, str(HERE / "golden"))
-from gen_inputs import checksum, dm_inputs, kmeans_inputs  # noqa: E402
+from gen_inputs import checksum, dm_inputs, kmeans_inputs, load_kmeans_golden  # noqa: E402
 
 from oracle import kmeans as ok  # noqa: E402
 
-_KM = HERE / "golden" / "kmeans_golden.npz"
-pytestmark = pytest.mark.skipif(not _KM.exists(), reason="kmeans_golden.npz not generated yet")
-GK = np.load(_KM) if _KM.exists() else None
+GK = load_kmeans_golden(HERE / "golden")
+pytestmark = pytest.mark.skipif(GK is None, reason="kmeans_golden*.npz not generated yet")
 
 
 def from_bits(a):
@@ -24,7 +23,7 @@ def from_bits(a):
 
 
 def _have(name):
-    return GK is not None and f"km_{name}_in" in GK.files
+    return GK is not None and f"km_{name}_in" in GK
 
 
 def _case(name):

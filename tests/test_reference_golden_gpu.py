@@ -19,14 +19,13 @@ pytestmark = pytest.mark.gpu
 
 HERE = Path(__file__).resolve().parent
 sys.path.insert(0, str(HERE / "golden"))
-from gen_inputs import checksum, dm_inputs, kmeans_inputs, smse_inputs  # noqa: E402
+from gen_inputs import checksum, dm_inputs, kmeans_inputs, load_kmeans_golden, smse_inputs  # noqa: E402
 
 BIG = ("hyq", "hyk", "wank")  # stored subsampled: every 4th token of the Lloyd-loop labels, every 4th centroid
 
 G1 = np.load(HERE / "golden" / "svg1_golden.npz")
-_KM = HERE / "golden" / "kmeans_golden.npz"
-GK = np.load(_KM) if _KM.exists() else None
-needs_km = pytest.mark.skipif(GK is None, reason="tests/golden/kmeans_golden.npz not generated yet")
+GK = load_kmeans_golden(HERE / "golden")
+needs_km = pytest.mark.skipif(GK is None, reason="tests/golden/kmeans_golden*.npz not generated yet")
 
 
 def from_bits(a, dtype=torch.bfloat16):
@@ -67,7 +66,7 @@ def test_sample_mse_matches_reference_processor(cuda, case):
 
 # ------------------------------------------------------------------------------------------------ flash k-means
 def _km_case(name):
-    if f"km_{name}_in" not in GK.files:
+    if f"km_{name}_in" not in GK:
         pytest.skip(f"golden case {name} not generated yet")
     seed, B, N, D, K, clustered, csum = GK[f"km_{name}_in"]
     x, init = kmeans_inputs(seed, int(B), int(N), int(D), int(K), int(clustered))
@@ -158,7 +157,7 @@ def test_kmeans_run_matches_reference_loop(cuda, name, iters):
     # K > number of blobs (several centroids compete inside one blob): Lloyd amplifies near-tie label noise, the
     # partition of a blob between its centroids drifts while the quality (inertia, above) stays the same
     assert moved <= (0.002 if well_conditioned else 0.6) * x.shape[0] * x.shape[1], moved
-    if f"km_{name}_run{iters}_labels" not in GK.files:
+    if f"km_{name}_run{iters}_labels" not in GK:
         return  # full-size cases keep labels / centroids of the 2-iteration run only
     stride = 4 if name in BIG else 1
     ref_lab = torch.from_numpy(GK[f"km_{name}_run{iters}_labels"].astype(np.int64))
@@ -254,7 +253,7 @@ def test_varblock_attention_matches_reference_flashinfer(cuda):
     """dynamic_block_sparse_fwd_flashinfer (svg/kmeans_utils.py:1319-1392, the reference's LIVE SVG2 kernel) output,
     recorded on a B200, vs svgb_attn_fwd on the same inputs; tolerance of the reference's own test
     (test_sparse_attn_dyn_blk_wan.py:133: atol = rtol = 1e-2)."""
-    if "fi_o" not in GK.files:
+    if "fi_o" not in GK:
         pytest.skip("FlashInfer golden unavailable: " + str(GK["fi_error"]))
     from svgb200 import kmeans_utils as ku
 
